@@ -15,6 +15,10 @@ Before the warm-up the MSM form is chosen by measurement on the key about to be 
 bb_groth16_autotune in a child process, at N > 1 by the collective tuner behind per-rank child probes; the timed steps
 run the chosen form only and the line records every form's milliseconds under `autotune` (--autotune 0: default form).
 
+--dump-outputs DIR writes what the last timed step returned (prove: the 192 proof bytes; msm: the point; ntt: the same
+fixed sample of 2^16 rows of the buffer after the forward transform and after the inverse that restores it) as
+DIR/<name>.npy, so that two builds can be compared output for output.
+
 The oracle (oracle/) is used only by the cpu_baseline leg and by --impl reference.
 """
 import argparse
@@ -45,7 +49,9 @@ def parse():
     ap.add_argument("--log-size", type=int, default=None, help="log2 of constraints (prove) / points (msm, ntt)")
     ap.add_argument("--cpu-sample-log", type=int, default=17, help="log2 constraints of the CPU baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--ref-budget-s", type=float, default=1200.0, help="--impl reference: wall-clock bound of the proving loop")
+    ap.add_argument("--ref-budget-s", type=float, default=None,
+                    help="--impl reference: optional wall-clock bound of the proving loop; when given it overrides --steps / --warmup, "
+                         "which shrink to fit it (the line reports what ran)")
     ap.add_argument("--window-bits", type=int, default=0)
     ap.add_argument("--precompute", type=int, default=None, help="force msm_precompute (0 = per-window bucket sets, 1 = window multiples + one bucket array "
                                                                    "per window, 2 = window multiples + ONE bucket array) instead of measuring")
@@ -68,7 +74,14 @@ def parse():
     ap.add_argument("--witness", default="uniform", choices=["uniform", "boolean"],
                     help="boolean: every second aux value is overwritten with 0/1 (SURVEY.md 8d config 2's boolean-heavy variant; "
                          "exercises the Exponent::Zero/One fast paths; no longer a satisfying assignment)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to this back-end's arm only")
+    return args
 
 
 T0 = time.time()
@@ -84,6 +97,30 @@ def emit(line):
 
 def log(msg):
     print(f"[bench +{time.time() - T0:7.1f}s] {msg}", file=sys.stderr, flush=True)
+
+
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SAMPLE_ROWS = 1 << 16
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each result as out_dir/<name>.npy: its bytes (proof bytes, little-endian limbs of field elements and
+    points) as float32, one value 0..255 per byte, which float32 holds exactly.  The inputs of every workload come
+    from fixed seeds, so two builds run with the same arguments must write identical files."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {name: np.frombuffer(np.ascontiguousarray(a).tobytes(), np.uint8).reshape(np.shape(a)[:-1] + (-1,)).astype(np.float32)
+           for name, a in arrays.items()}
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise ValueError(f"{total} bytes of outputs exceed the {DUMP_MAX_BYTES}-byte dump limit")
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"outputs written to {out_dir}: " + ", ".join(f"{k} {v.shape}" for k, v in out.items()))
+
+
+def sample_rows(n, k=DUMP_SAMPLE_ROWS):
+    """a fixed, seeded choice of min(n, k) row indices of an n-row output, ascending"""
+    return np.arange(n) if n <= k else np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
 
 
 def measured_traffic():
@@ -243,8 +280,8 @@ def run_reference(args):
     """The reference arm: the restated bellman CPU prover (oracle-1; the Rust crate cannot be built in
     this image) on the SAME workload as the GPU arm -- the 2^20-constraint MiMC chain unless
     --log-size says otherwise -- with the same --steps / --warmup, on the host threads this process
-    may use.  --ref-budget-s bounds the leg: if the box is too slow for K+W proves inside it, the
-    warm-up and then the step count shrink and the line reports what ran."""
+    may use.  Only when --ref-budget-s is given does it bound the leg: if K+W proves do not fit inside
+    it, the warm-up and then the step count shrink and the line reports what ran."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
@@ -487,6 +524,8 @@ def run_prove(args):
             proof_single = bb.create_proof(asg, full, r, s, dev)
             full.free()
             assert proof_single == proof_val, "sharded proof differs from the single-GPU proof"
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"proof": np.frombuffer(proof_val, np.uint8)})
     n_constraints = shape["num_constraints"]
     value = n_constraints * args.steps / dt_val
     e2e = n_constraints * args.steps / dt_e2e
@@ -680,6 +719,8 @@ def run_msm(args):
     want = bb.fixed_base_mul(worker, bb.G1, dot.reshape(1, 4), form=bb.FORM_CANONICAL)
     line["config"]["result_check"] = "msm == [sum k_i e_i]G (device Fr inner product + fixed-base multiplication): " + \
         ("equal" if np.array_equal(np.asarray(out).reshape(-1), np.asarray(want).reshape(-1)) else "MISMATCH")
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"msm": np.asarray(out)})
     emit(line)
     assert line["config"]["result_check"].endswith("equal"), "MSM result differs from [sum k_i e_i]G"
     worker.close()
@@ -713,6 +754,14 @@ def run_ntt(args):
     back = np.zeros_like(v)
     worker.download(d, back)
     ok = bool(np.array_equal(back, v))                      # domain.rs:444-450 round trip, bit exact
+    if args.dump_outputs:
+        # a step hands back its input (forward, then inverse), so the last step's forward result is computed once more,
+        # untimed, from the buffer the step restored: bit for bit the same input whenever the round trip is exact
+        rows = sample_rows(n)
+        bb.ntt_device(worker, d, log_n, bb.NTT_FFT)
+        fwd = np.zeros_like(v)
+        worker.download(d, fwd)
+        dump_outputs(args.dump_outputs, {"ntt": back[rows], "ntt_forward": fwd[rows]})
     hbm_peak, peak_src = peaks()
     achieved = 2 * 64.0 * n * args.steps / dt / 1e9        # 64 B per point per transform (SURVEY.md 8d)
     line = {"metric": "fr_ntt_mpt_per_sec", "value": 2 * n * args.steps / dt / 1e6, "unit": "Mpt/s (forward+inverse counted as 2n points)",

@@ -7,6 +7,7 @@ import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+NO_CUDA = {"CUDA_VISIBLE_DEVICES": ""}          # a tuner child of the real library finds no device, GPU or not
 REQUIRED = {"impl", "metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better",
             "scaling", "vs_baseline", "dtype", "data", "config", "cpu_baseline", "e2e"}
 
@@ -67,7 +68,8 @@ def test_own_arm_dry_run_on_the_emulated_device(tmp_path, emu_lib):
     to end with the CUDA library replaced by the host-fiber build of the same sources and torch.cuda
     stubbed: checks the script and the JSON contract, not the numbers."""
     script = tmp_path / "dry.py"
-    script.write_text(f"ROOT = {ROOT!r}\nEMU_LIB = {emu_lib!r}\nEXTRA = []\n" + DRY_RUN)
+    dump = tmp_path / "outputs"
+    script.write_text(f"ROOT = {ROOT!r}\nEMU_LIB = {emu_lib!r}\nEXTRA = ['--dump-outputs', {str(dump)!r}]\n" + DRY_RUN)
     res = subprocess.run([sys.executable, str(script)], capture_output=True, text=True, timeout=900, cwd=ROOT)
     assert res.returncode == 0, res.stderr[-3000:]
     lines = [l for l in res.stdout.splitlines() if l.strip()]
@@ -85,12 +87,18 @@ def test_own_arm_dry_run_on_the_emulated_device(tmp_path, emu_lib):
     assert "workload" in d["config"] and "model" not in d["config"]
     at = d["autotune"]                                  # the MSM form was measured before the warm-up; every form eligible here
     assert len(at["ms"]) == len(at["forms"]) >= 2 and all(t > 0 for t in at["ms"]) and at["ms"][at["chosen"]] == min(at["ms"])
+    import hashlib
+    import numpy as np
+    assert sorted(os.listdir(dump)) == ["proof.npy"]      # the last timed step's proof, byte values as float32
+    proof = np.load(dump / "proof.npy")
+    assert proof.dtype == np.float32 and proof.shape == (192,)
+    assert hashlib.sha256(proof.astype(np.uint8).tobytes()).hexdigest() == d["proof_sha256"]
 
 
 def test_tuner_child_mode_and_parent_fallback(tmp_path, emu_lib):
     """bench.py's sandboxed tuner: (1) child mode (--tune-child) builds the key and witness, tunes and prints its report --
-    run here on the emulated device; (2) a parent whose child cannot run (the real library finds no CUDA device in this
-    container) records the error and measures the default form."""
+    run here on the emulated device; (2) a parent whose child cannot run (the real library finds no CUDA device: none is
+    made visible) records the error and measures the default form."""
     # (the unsharded tuner itself runs in the dry run above; here) the child of rank 1 of 2 -- the gate in front of the
     # collective tuner: that rank's key shard, no process group
     script = tmp_path / "child_shard.py"
@@ -102,7 +110,7 @@ def test_tuner_child_mode_and_parent_fallback(tmp_path, emu_lib):
     assert all(t > 0 for t in rep["ms"]) and rep["name"]
     script = tmp_path / "parent.py"
     script.write_text(f"ROOT = {ROOT!r}\nEMU_LIB = {emu_lib!r}\nEXTRA = ['--autotune', '1', '--no-cpu-baseline']\n" + DRY_RUN)
-    res = subprocess.run([sys.executable, str(script)], capture_output=True, text=True, timeout=900, cwd=ROOT)
+    res = subprocess.run([sys.executable, str(script)], capture_output=True, text=True, timeout=900, cwd=ROOT, env=dict(os.environ, **NO_CUDA))
     assert res.returncode == 0, res.stderr[-3000:]
     d = json.loads([l for l in res.stdout.splitlines() if l.strip()][-1])
     at = d["autotune"]
@@ -112,11 +120,11 @@ def test_tuner_child_mode_and_parent_fallback(tmp_path, emu_lib):
 
 def test_own_arm_dry_run_two_ranks(tmp_path, emu_lib):
     """bench.py --gpus 2 under torchrun with gloo and the emulated device: the sharded step, the max over ranks, the gate in
-    front of the collective tuner (the per-rank tuner children cannot run here -- no CUDA device -- so both ranks must stay on
-    the default form and say why), the sharded proof == single-GPU proof check, one JSON line from rank 0."""
+    front of the collective tuner (the per-rank tuner children cannot run here -- no CUDA device is made visible -- so both
+    ranks must stay on the default form and say why), the sharded proof == single-GPU proof check, one JSON line from rank 0."""
     script = tmp_path / "dry2.py"
     script.write_text(f"ROOT = {ROOT!r}\nEMU_LIB = {emu_lib!r}\nEXTRA = ['--gpus', '2', '--autotune', '1', '--no-cpu-baseline']\n" + DRY_RUN)
-    env = dict(os.environ, BB_BENCH_DIST_BACKEND="gloo")
+    env = dict(os.environ, BB_BENCH_DIST_BACKEND="gloo", **NO_CUDA)
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2", "--master-addr", "127.0.0.1",
            "--master-port", "29541", str(script)]
     res = subprocess.run(cmd, capture_output=True, text=True, timeout=900, cwd=ROOT, env=env)
@@ -135,12 +143,18 @@ def test_msm_microbench_dry_run_on_the_emulated_device(tmp_path, emu_lib):
     """bench.py --workload msm (BASELINE configs[2] shape, here 2^10 points): both MSM forms are measured, the result
     is asserted against [sum k_i e_i]G inside the script"""
     script = tmp_path / "dry_msm.py"
-    script.write_text(f"ROOT = {ROOT!r}\nEMU_LIB = {emu_lib!r}\nEXTRA = ['--workload', 'msm', '--log-size', '10']\n" + DRY_RUN)
+    dump = tmp_path / "outputs"
+    script.write_text(f"ROOT = {ROOT!r}\nEMU_LIB = {emu_lib!r}\nEXTRA = ['--workload', 'msm', '--log-size', '10', '--dump-outputs', {str(dump)!r}]\n"
+                      + DRY_RUN)
     res = subprocess.run([sys.executable, str(script)], capture_output=True, text=True, timeout=900, cwd=ROOT)
     assert res.returncode == 0, res.stderr[-3000:]
     d = json.loads([l for l in res.stdout.splitlines() if l.strip()][0])
     assert d["metric"] == "g1_msm_mpt_per_sec" and d["config"]["result_check"].endswith("equal")
     assert len(d["autotune"]["ms"]) == 2 and all(t > 0 for t in d["autotune"]["ms"])
+    import numpy as np
+    point = np.load(dump / "msm.npy")                     # the G1 point of the last timed step: 12 limbs, 96 bytes
+    assert point.dtype == np.float32 and point.shape == (1, 96)
+    assert point[0, :16].astype(np.uint8).tobytes().hex() == d["result_head"]
 
 
 def test_reference_arm_sizes_its_pool_to_the_cpu_quota(monkeypatch):
@@ -171,3 +185,42 @@ def test_reference_arm_sizes_its_pool_to_the_cpu_quota(monkeypatch):
     assert bench.host_cpu_info()["threads"] == 3
     monkeypatch.setenv("BB_ORACLE_THREADS", "5")
     assert bench.host_cpu_info()["threads"] == 5
+
+
+def test_ntt_microbench_dump_on_the_emulated_device(tmp_path, emu_lib):
+    """bench.py --workload ntt --dump-outputs: the buffer after the last timed step's forward transform and after its
+    inverse (here all 2^10 rows; a fixed sample of 2^16 rows at larger sizes), bytes as float32.  The forward rows must
+    be the oracle's transform of the seed-41 input, the restored rows that input."""
+    script = tmp_path / "dry_ntt.py"
+    dump = tmp_path / "outputs"
+    script.write_text(f"ROOT = {ROOT!r}\nEMU_LIB = {emu_lib!r}\nEXTRA = ['--workload', 'ntt', '--log-size', '10', '--dump-outputs', {str(dump)!r}]\n"
+                      + DRY_RUN)
+    res = subprocess.run([sys.executable, str(script)], capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert res.returncode == 0, res.stderr[-3000:]
+    d = json.loads([l for l in res.stdout.splitlines() if l.strip()][0])
+    assert d["metric"] == "fr_ntt_mpt_per_sec" and d["steps"] == 2 and d["config"]["round_trip_bit_exact"] is True
+    import numpy as np
+    import bellman_b200 as bb
+    from oracle import o1
+    n = 1 << 10
+    saved = (bb.LIB_PATH, bb._lib)
+    bb.LIB_PATH, bb._lib = emu_lib, None              # bench.py's input: the seed-41 scalars of the device generator
+    try:
+        w = bb.Worker(0)
+        dv = w.device_alloc(n * 32)
+        bb.synth_scalars_device(w, 41, n, dv)
+        v = np.zeros((n, 4), np.uint64)
+        w.download(dv, v)
+        w.device_free(dv)
+        w.close()
+    finally:
+        bb.LIB_PATH, bb._lib = saved
+    assert sorted(os.listdir(dump)) == ["ntt.npy", "ntt_forward.npy"]
+
+    def limbs(name):
+        a = np.load(dump / name)
+        assert a.dtype == np.float32 and a.shape == (n, 32) and a.max() <= 255 and np.array_equal(a, np.round(a))
+        return a.astype(np.uint8).view(np.uint64)
+
+    assert np.array_equal(limbs("ntt_forward.npy"), o1.fft(v, o1.FFT))
+    assert np.array_equal(limbs("ntt.npy"), v)
