@@ -9,6 +9,8 @@ import numpy as np
 import bellman_b200 as bb
 from oracle import o1
 
+import test_gpu_points as GP
+
 R = o1.FR_MODULUS
 
 
@@ -48,3 +50,19 @@ def test_point_add_mul_compress_host():
         for i in range(len(ks)):
             assert bb.point_compress(group, pts[i:i + 1]) == bytes(want[i])
         assert bb.point_compress(group, zero) == bytes([0xC0] + [0] * (47 if group == bb.G1 else 95))
+        # points outside the prime-order subgroup (a key read unchecked may hold them): small-order points T and P + T,
+        # against exact integer arithmetic.  For T of order 3 the ladder's table entries 3T, 9T, 15T are the identity.
+        cv = GP._curve(group)
+        p_int = GP.subgroup_point(group, 3)
+        odd = [GP.torsion_point(group, ell, 6) for ell in GP.ORDERS[group]]
+        odd += [cv.add(p_int, t) for t in odd] + [GP.random_curve_point(group, random.Random(6))]
+        for a in odd:
+            a_arr = GP.to_abi(group, [a])
+            for b in odd[:4] + [a, cv.neg(a), p_int, None]:
+                assert GP.from_abi(group, bb.point_add(group, a_arr, GP.to_abi(group, [b])))[0] == cv.add(a, b)
+            for k in [0, 1, 2, 3, 15, 16, 17, 31, 32, 33, R - 1, R - 2] + [rng.randrange(R) for _ in range(3)]:
+                out = np.zeros((1, w), np.uint64)
+                kc = o1.fr_to_canonical(o1.fr_from_ints([k]))
+                assert lib.bb_point_mul(C.c_int(group), a_arr.ctypes.data_as(C.c_void_p), kc.ctypes.data_as(C.c_void_p),
+                                        C.c_int(bb.FORM_CANONICAL), out.ctypes.data_as(C.c_void_p)) == 0
+                assert GP.from_abi(group, out)[0] == GP.mul_exact(group, a, k), k
